@@ -2,6 +2,7 @@
 """bench.py -- Mrays/s of the PathIntegrator hot path on N B200s (BASELINE.json metric).
 
     python bench.py --gpus N --steps K --warmup W [--workload statue|cornell|conference|landscape|landscape-64|cornell-textured|cornell-direct|cornell-whitted|cornell-ao] [--impl reference]
+    [--dump-outputs DIR]
 
 A "step" is one full frame of the workload rendered through the wavefront kernels.  The default workload is
 BASELINE.json configs[2] -- the Ganesha stand-in (4.31 M triangles, path integrator, 128 spp, 1024x1024), the largest
@@ -203,9 +204,14 @@ def run_reference(args):
     print(json.dumps(line))
 
 
-def measure(args, name, steps, warmup, dist, rank, world, local, want_cpu):
+RAY_COUNTERS = ("camera_rays", "rays", "closest_rays", "shadow_rays")
+
+
+def measure(args, name, steps, warmup, dist, rank, world, local, want_cpu, dump_dir=None):
     """One workload through the contract: K device-resident steps, K end-to-end steps, the per-kernel pass.  Returns the JSON
-    line (rank 0) or None."""
+    line (rank 0) or None.  `dump_dir`: rank 0 writes there what the last device-resident step handed its caller -- the
+    frame's film (film.npy, float32 H x W x 4, reduced over the ranks) and the stats' ray counters (ray_counters.npy, float64,
+    RAY_COUNTERS order, summed over the ranks)."""
     import numpy as np
     import torch
 
@@ -281,6 +287,12 @@ def measure(args, name, steps, warmup, dist, rank, world, local, want_cpu):
         dist.all_reduce(tot, op=dist.ReduceOp.SUM)
     ms_total = float(ms.item())
     rays_total = float(tot[0].item())
+    outputs = None
+    if dump_dir is not None:
+        last = torch.tensor([float(st[k]) for k in RAY_COUNTERS], device="cuda", dtype=torch.float64)
+        if dist is not None:
+            dist.all_reduce(last, op=dist.ReduceOp.SUM)
+        outputs = {"film": film.cpu().numpy(), "ray_counters": last.cpu().numpy()}
     # ---- timed: K steps end to end (host buffers) ------------------------------------------------
     # The step's inputs live in pinned host memory, as the bench contract asks (the caller's scene arrays are page-locked once, here,
     # through pbrt_gpu_host_register; pbrt_gpu_scene_create then DMAs them where they lie).
@@ -352,6 +364,11 @@ def measure(args, name, steps, warmup, dist, rank, world, local, want_cpu):
         sync_all()
     if rank != 0:
         return None
+    if outputs is not None:
+        assert sum(a.nbytes for a in outputs.values()) <= 64 << 20  # every workload's film is at most 1920 x 1080 x 4 floats
+        os.makedirs(dump_dir, exist_ok=True)
+        for k, a in outputs.items():
+            np.save(os.path.join(dump_dir, k + ".npy"), a)
     nodes_v, tris_t, rays_frame, cam_frame, slots_frame, verts_frame = (float(x) for x in cnt.tolist())
     trace_ms = float(ser[0].item()) / world  # mean over ranks of one frame's k_trace time (single-stream pass)
     shade_ms = float(ser[1].item()) / world
@@ -461,7 +478,10 @@ def main():
     ap.add_argument("--small", action="store_true", help="debug: smaller statue mesh")
     ap.add_argument("--no-inproc", dest="inproc", action="store_false", help="N > 1: skip the pbrt_gpu_render_multi (one process, N devices) leg")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the film and ray counters of the last timed step of --workload as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.steps < 1 or args.impl != "ours"):
+        ap.error("--dump-outputs needs --steps >= 1 and --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -480,7 +500,7 @@ def main():
 
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-    line = measure(args, args.workload, args.steps, args.warmup, dist, rank, world, local, want_cpu=not args.no_cpu)
+    line = measure(args, args.workload, args.steps, args.warmup, dist, rank, world, local, want_cpu=not args.no_cpu, dump_dir=args.dump_outputs)
     if args.workload == "statue" and not args.no_extra:
         # BASELINE.json configs[1] (round 1's default) in short form, so that the driver's records keep a Cornell number
         ex = measure(args, "cornell", min(args.steps, 3), 3, dist, rank, world, local, want_cpu=False)
